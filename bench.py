@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- feature frames/s of the CtuCopy hot path on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--utts U] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--utts U] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of synthetic 16 kHz utterances
 (10 000 x 10 s per GPU by default = 9.98 M frames, SURVEY.md 8(d) throughput set; inputs
@@ -328,6 +328,7 @@ def main():
                     help="the other BASELINE configs under 'workloads': auto = all of them on one GPU, PLP only under torchrun")
     ap.add_argument("--no-selfcheck", action="store_true")
     ap.add_argument("--cli-utts", type=int, default=20000, help="10 s files for the file -> file run of the command-line host (0 = skip)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a seeded sample of the last timed step's output to DIR/*.npy (rank 0's shard under torchrun)")
     a = ap.parse_args()
     a.warmup = max(a.warmup, 3) if a.impl == "ours" else a.warmup
     if a.impl == "reference":
@@ -386,7 +387,23 @@ def main():
     torch.cuda.synchronize()
     stream = torch.cuda.current_stream().cuda_stream
 
-    def measure(workload, steps, warmup, e2e_steps, with_clocks, check):
+    def dump_outputs(d, plan, d_out, sig, lens):
+        """The output of the last timed step as a caller receives it, for comparing two builds output for output: a fixed,
+        seeded sample of whole utterances (features [utt, frame, dim] or waveform [utt, sample], float32) within 64 MB,
+        and the batch positions of the sampled utterances (float64).  An utterance larger than the whole budget is cut to
+        its leading rows."""
+        os.makedirs(d, exist_ok=True)
+        off = plan.wave_offsets if sig else plan.row_offsets
+        budget = (60 << 20) // (4 * (1 if sig else d_out.shape[1]))          # rows of float32 within 60 MiB
+        longest = max(int(off[i + 1] - off[i]) for i in range(len(lens)))
+        k = min(len(lens), 256, max(1, budget // longest))
+        keep = min(longest, budget // k)
+        sel = np.sort(np.random.default_rng(0).choice(len(lens), k, replace=False))
+        rows = [d_out[int(off[i]): min(int(off[i + 1]), int(off[i]) + keep)].float().cpu().numpy() for i in sel]
+        np.save(os.path.join(d, "waveform.npy" if sig else "features.npy"), np.stack(rows))
+        np.save(os.path.join(d, "utterances.npy"), sel.astype(np.float64))
+
+    def measure(workload, steps, warmup, e2e_steps, with_clocks, check, dump=None):
         args, bytes_step, flops = WORKLOADS[workload]
         hd = cb.Handle(args, device=local)
         plan = hd.plan(lens)
@@ -430,6 +447,8 @@ def main():
         hd.profile(False)
         clocks = sampler.stop(t_begin, t_end) if sampler else None
         ms = max_over_ranks(ms)
+        if dump and rank == 0:
+            dump_outputs(dump, plan, d_out, sig, lens)
         # per-kernel average duration over the timed region; the dominant kernel is the one with the largest share
         by = {}
         for n, t in recs:
@@ -512,7 +531,7 @@ def main():
                 "kernels": r["kinfo"]}
 
     check = not a.no_selfcheck
-    r = measure(a.workload, a.steps, a.warmup, a.e2e_steps, True, check)
+    r = measure(a.workload, a.steps, a.warmup, a.e2e_steps, True, check, a.dump_outputs)
     value = world * r["frames"] * a.steps / (r["ms"] / 1000.0)
     roof = roofline_of(a.workload, r, value)
     if roof:

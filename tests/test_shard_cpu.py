@@ -1,15 +1,14 @@
 """Host-side multi-GPU logic on CPU: list partitioning and the ordered merge of per-rank
-containers (SURVEY.md 8e).  The per-rank containers are produced by the REFERENCE binary
-(oracle/_ref, test infrastructure) on each rank's list range, so the check is exact: the
-merged ark+scp / pfile must equal, byte for byte, what the reference writes for the whole
-list in one process.  A world_size-2 gloo run covers the plumbing bench.py uses under
+containers (SURVEY.md 8e).  The per-rank containers are the ones one process writes for each
+rank's list range, stored in tests/golden/shard_containers.npz (tests/golden/make_shard_golden.py),
+so the check is exact: the merged ark+scp / pfile must equal, byte for byte, what one process
+writes for the whole list.  A world_size-2 gloo run covers the plumbing bench.py uses under
 torchrun (rank ranges, barrier, max-over-ranks, gather to rank 0)."""
 import os
 import subprocess
 import sys
 
 import numpy as np
-import pytest
 
 import golden_util as gu
 import ref_runner as rr
@@ -18,7 +17,6 @@ from ctucopy_b200 import shard
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 EXE = os.path.join(ROOT, "host", "ctucopy_b200")
 B = ["-fs", "16000", "-format_in", "raw", "-dither", "0"]
-needs_ref = pytest.mark.skipif(rr.ref_binary("O2") is None, reason="oracle/_ref not built")
 
 
 def test_partition_is_contiguous_balanced_and_total():
@@ -36,37 +34,42 @@ def test_partition_is_contiguous_balanced_and_total():
     assert shard.split_ext_vad(ev, [3, 3, 4], [0, 2, 3]) == [ev[:6], ev[6:]]
 
 
-def _ref_containers(args, utts, d, tag):
-    """reference binary on `utts` -> (ark, scp, pfile) bytes, container paths under d/tag"""
-    os.makedirs(os.path.join(d, tag), exist_ok=True)
-    lst = os.path.join(d, tag, "list.scp")
-    with open(lst, "w") as fh:
-        for name, u in utts:
-            p = os.path.join(d, name + ".raw")
-            if not os.path.exists(p):
-                np.asarray(u).astype("<i2").tofile(p)
-            fh.write("%s %s\n" % (p, name))
-    out = {}
-    for kind in ("ark", "pfile"):
-        tgt = os.path.join(d, tag, "o." + kind)
-        a = B + args + ["-format_out", "%s=%s" % (kind, tgt), "-S", lst]
-        pr = subprocess.run([rr.ref_binary("O2")] + a, capture_output=True, cwd=d)
-        assert pr.returncode == 0, pr.stderr.decode()
-        out[kind] = open(tgt, "rb").read()
-    out["scp"] = open(os.path.join(d, tag, "o.scp")).read()
+def _containers(name, tag, d):
+    """stored containers of list `name` (make_shard_golden.SHARD_LISTS) for `tag` -> (ark, scp, pfile) bytes, scp paths under d"""
+    z = np.load(os.path.join(gu.GOLDEN, "shard_containers.npz"))
+    out = {kind: z["%s_%s_%s" % (name, tag, kind)].tobytes() for kind in ("ark", "pfile")}
+    out["scp"] = z["%s_%s_scp" % (name, tag)].tobytes().decode().replace("{D}", d)
     return out
 
 
-@needs_ref
+def test_stored_containers_hold_the_reference_matrices(tmp_path):
+    """The stored plpc containers against what the reference wrote for each utterance with the same options (the plpc_ark
+    golden, one utterance per run): same keys in list order, the same matrix header bytes at every scp offset, matrices
+    within the parity tolerance."""
+    c = gu.Case("plpc_ark")
+    whole = _containers("plpc", "whole", str(tmp_path))
+    got = rr.parse_ark(whole["ark"])
+    order = (0, 4, 1, 5, 2, 3)
+    assert list(got) == ["utt%d" % i for i in order]
+    offs = [int(ln.rsplit(":", 1)[1]) for ln in whole["scp"].splitlines()]
+    for i, off in zip(order, offs):
+        ref_off = int(c.aux[i].decode().split()[1].rsplit(":", 1)[1])
+        assert whole["ark"][off:off + 15] == c.raw[i][ref_off:ref_off + 15], i
+        a, b = got["utt%d" % i], c.payload(i)
+        assert a.shape == b.shape and np.all(np.abs(a - b) <= 1e-4 * np.abs(b) + 1e-3), i
+
+
 def test_merged_containers_equal_the_single_process_reference(tmp_path):
     d = str(tmp_path)
     ins = gu.inputs()
     utts = [("utt%d" % i, ins[i]) for i in (0, 4, 1, 5, 2, 3)]
     args = ["-preset", "mfcc", "-preem", "0.97"]
-    whole = _ref_containers(args, utts, d, "whole")
+    whole = _containers("mfcc", "whole", d)
     for world in (2, 3):
         cut = shard.partition([len(u) for _, u in utts], world)
-        parts = [_ref_containers(args, utts[cut[r]:cut[r + 1]], d, "w%dr%d" % (world, r)) for r in range(world)]
+        parts = [_containers("mfcc", "w%dr%d" % (world, r), d) for r in range(world)]
+        for r, p in enumerate(parts):
+            assert [ln.split()[0] for ln in p["scp"].splitlines()] == [n for n, _ in utts[cut[r]:cut[r + 1]]]
         # python merge
         assert shard.merge_pfile([p["pfile"] for p in parts]) == whole["pfile"]
         scps = [p["scp"].replace("/w%dr%d/" % (world, r), "/whole/") for r, p in enumerate(parts)]
@@ -103,7 +106,8 @@ ins = gu.inputs()
 utts = [("utt%%d" %% i, ins[i]) for i in (0, 4, 1, 5, 2, 3)]
 lo, hi = shard.rank_range([len(u) for _, u in utts], rank, world)
 d = sys.argv[1]
-part = T._ref_containers(["-preset", "plpc"], utts[lo:hi], d, "r%%d" %% rank)
+part = T._containers("plpc", "r%%d" %% rank, d)
+assert [ln.split()[0] for ln in part["scp"].splitlines()] == [n for n, _ in utts[lo:hi]]
 part["scp"] = part["scp"].replace("/r%%d/" %% rank, "/whole/")
 dist.barrier()
 t = torch.tensor([float(rank + 1)], dtype=torch.float64)
@@ -112,7 +116,7 @@ assert t.item() == world
 gathered = [None] * world if rank == 0 else None
 dist.gather_object(part, gathered, dst=0)
 if rank == 0:
-    whole = T._ref_containers(["-preset", "plpc"], utts, d, "whole")
+    whole = T._containers("plpc", "whole", d)
     assert shard.merge_pfile([g["pfile"] for g in gathered]) == whole["pfile"]
     ark, scp = shard.merge_ark([g["ark"] for g in gathered], [g["scp"] for g in gathered])
     assert ark == whole["ark"] and scp == whole["scp"]
@@ -121,7 +125,6 @@ dist.destroy_process_group()
 """
 
 
-@needs_ref
 def test_world_size_2_gloo_shards_merge_to_the_single_process_result(tmp_path):
     script = tmp_path / "worker.py"
     script.write_text(WORKER % {"root": ROOT})
