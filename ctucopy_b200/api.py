@@ -239,8 +239,7 @@ class Handle:
         return int(self.L.ctu_launch_count(self.h))
 
     def set_option(self, name: str, value: int):
-        """Run-time knobs outside the reference's option set (ctu_set_option): copy_only, chunk_mb, split_front,
-        synth_from_pcm."""
+        """Run-time knobs outside the reference's option set (ctu_set_option): copy_only, chunk_mb."""
         self._check(self.L.ctu_set_option(self.h, name.encode(), int(value)))
 
     def profile(self, on: bool):

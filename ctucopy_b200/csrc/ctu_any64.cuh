@@ -1,7 +1,7 @@
 // fp64 building blocks of the GENERAL kernels (FFT sizes other than 512): one warp owns a frame, the transform is an
 // in-place FFT (radix-4 passes) of nfft/2 complex points in shared memory.  Used by the general synthesis (ctu_synth_any.cuh) and
 // by the general Burg front end below.  Speed is secondary here (every BASELINE configuration takes the 512-point
-// kernels); the arithmetic conventions are those of k_synth / k_burg, restated from the same reference lines.
+// kernels); the arithmetic conventions are those of k_synth_c / k_burg, restated from the same reference lines.
 #ifndef CTU_ANY64_CUH
 #define CTU_ANY64_CUH
 

@@ -111,8 +111,6 @@ struct ctu_handle {
     // run-time knobs outside the reference's option set (ctu_set_option; the environment gives the defaults)
     int copy_only = 0;                   // host entry points: copies only, kernels skipped (control measurement)
     int chunk_mb = 32;                   // MB of PCM per pipeline chunk of the host entry points
-    int split_front = 1;                 // 1: PCM -> spectrum -> features as two kernels; 0: the single fused kernel
-    int synth_from_pcm = 0;              // 1: synthesis recomputes the forward transform instead of reading the stored X
     int fuse_nr = 1;                     // 1: the noise-reduction scan runs inside k_bank (tile in shared memory) where it can
     int front256 = 1;                    // 1: 256-point frames take k_frames256 for PCM -> spectrum; 0: the general kernel throughout
     int compact_static = 1;              // 1: cepstra behind a delta chain are written as compact rows and the delta kernel writes the whole output row
@@ -718,8 +716,6 @@ int ctu_create(const ctu_config *cfg, int device, ctu_handle **out) {
     ctu_handle *h = new ctu_handle;
     h->cfg = *cfg;
     h->device = device;
-    if (const char *e = getenv("CTU_SPLIT_FRONT")) h->split_front = atoi(e);
-    if (getenv("CTU_SYNTH_FROM_PCM")) h->synth_from_pcm = 1;
     if (const char *e = getenv("CTU_FUSE_NR")) h->fuse_nr = atoi(e);
     if (const char *e = getenv("CTU_FRONT256")) h->front256 = atoi(e);
     if (const char *e = getenv("CTU_COMPACT_STATIC")) h->compact_static = atoi(e);
@@ -978,19 +974,15 @@ int ctu_plan_create(ctu_handle *h, const int64_t *off, int32_t n, ctu_plan **out
         return CTU_OK;
     }
     const bool nr_on = h->nr_mode != NR_NONE;
-    // PCM -> spectrum (k_frames2, 4-5 CTAs per SM) followed by spectrum -> features is faster than the single fused kernel
-    // (2 CTAs per SM) even though the spectrum then makes a round trip through HBM -- measured 12.4 -> 11.4 ms (MFCC_0_D_A),
-    // 12.6 -> 11.8 (PLP), 14.9 -> 14.1 (TRAP-DCT) per 9.98 M frames; CTU_SPLIT_FRONT=0 restores the fused kernel
-    const int split_front = h->split_front;
+    // the fp32 512-point feature chains always go PCM -> spectrum (k_frames2) -> k_bank
     const bool need_spec = h->signal_out || (nr_on && h->cfg.nr_when == 0) || (h->do_vad && h->vad_cri != VCRI_CEPDIST_FEA) ||
-                           (split_front && !h->precise && !h->generic && h->fea_kind != FEA_NONE) ||
+                           (!h->precise && !h->generic && h->fea_kind != FEA_NONE) ||
                            (fast256(h) && !h->precise && h->fea_kind != FEA_NONE);
     const bool lpc_kind = (h->fea_kind == FEA_LPA || h->fea_kind == FEA_LPC);
     const bool need_fb = !h->signal_out && ((nr_on && h->cfg.nr_when == 1) || lpc_kind);
     if (need_spec && (st = dev_alloc(h, p, &p->d_spec, (size_t)rows * h->spitch))) { ctu_plan_destroy(p); return st; }
     if (h->signal_out && h->bp.nfft && (st = dev_alloc(h, p, &p->d_yt, (size_t)rows * h->cfg.window))) { ctu_plan_destroy(p); return st; }
-    const int want_cspec = h->synth_from_pcm ? 0 : 1;
-    if (h->signal_out && !h->bp.nfft && want_cspec && (st = dev_alloc(h, p, &p->d_cspec, (size_t)rows * NBIN))) { ctu_plan_destroy(p); return st; }
+    if (h->signal_out && !h->bp.nfft && (st = dev_alloc(h, p, &p->d_cspec, (size_t)rows * NBIN))) { ctu_plan_destroy(p); return st; }
     if (need_fb && !h->precise && (st = dev_alloc(h, p, &p->d_fb, (size_t)rows * h->fb.nb))) { ctu_plan_destroy(p); return st; }
     if (need_fb && h->precise && (st = dev_alloc(h, p, &p->d_fb64, (size_t)rows * h->fb.nb))) { ctu_plan_destroy(p); return st; }
     if (h->do_vad && h->vad_cri == VCRI_CEPDIST_FEA && (st = dev_alloc(h, p, &p->d_fea64, (size_t)rows * h->feature_dim))) { ctu_plan_destroy(p); return st; }
@@ -1055,23 +1047,17 @@ static Range make_range(const ctu_plan *p, int u0, int u1) {
 }
 
 struct Range;
-// tile lists of one contiguous run of utterances for the two frame-kernel generations
+// tile list of one contiguous run of utterances for the frame kernels
 struct FrameTiles {
-    const int2 *t32; int64_t n32;     // 32-frame tiles (k_frames)
-    const int2 *t16; int64_t n16;     // 16-frame tiles (k_frames2)
+    const int2 *t16; int64_t n16;     // 16-frame tiles
     float2 *cplx = nullptr;           // PCM -> spectrum: also store the complex spectrum here (synthesis)
 };
 
-// Two generations of the fused frame kernel are kept because they bind on different things
-// (profiles/): k_frames (32-frame spectrum tile, lane = frame filter bank: fewest shared-memory
-// wavefronts, 2 CTAs/SM) wins whenever a filter bank follows; k_frames2 (group-local, 6
-// CTAs/SM) wins for PCM -> spectrum, where nothing follows the transform inside the kernel.
 template <int SRC, int DST, int KIND, int WT>
 static int launch_frames_w(ctu_handle *h, const FrameParams &P, const ctu_plan *p, const FrameTiles &ft, const int16_t *pcm,
                            const float *src, float *dst, cudaStream_t s) {
-    static const char *const names[3][3] = {{"k_frames<pcm,spec>", "k_frames<pcm,fb>", "k_frames<pcm,fea>"},
-                                            {"k_frames<spec,spec>", "k_frames<spec,fb>", "k_frames<spec,fea>"},
-                                            {"k_frames<fb,spec>", "k_frames<fb,fb>", "k_frames<fb,fea>"}};
+    static const char *const names[2][3] = {{"k_frames<pcm,spec>", "k_frames<pcm,fb>", "k_frames<pcm,fea>"},
+                                            {"k_frames<spec,spec>", "k_frames<spec,fb>", "k_frames<spec,fea>"}};
     if constexpr (SRC == SRC_PCM && DST == DST_SPEC) {
         if (fast256(h) && !P.dither && !P.dc1) {
             if (ft.n16 <= 0) return CTU_OK;
@@ -1121,28 +1107,12 @@ static int launch_frames_w(ctu_handle *h, const FrameParams &P, const ctu_plan *
         h->lc.begin(names[SRC][DST], s);
         kern<<<grid, F2_THREADS, bytes, s>>>(P, bd, tb, pcm, dst, (int)ft.n16, ft.cplx);
         h->lc.end(s);
-    } else if constexpr (SRC == SRC_SPEC) {
-        // 512-point spectra (rows of SPITCH floats) are consumed by k_bank (ctu_bank.cuh)
-        return fail(h, CTU_ERR_CONFIG, "CTU: internal: spectrum source outside k_bank");
+        CK(cudaGetLastError());
+        return CTU_OK;
     } else {
-        if (ft.n32 <= 0) return CTU_OK;
-        SmemLayout L = smem_layout(P.window, P.wshift, P.nb, SRC == SRC_PCM);
-        size_t bytes = (size_t)L.total * sizeof(float);
-        auto kern = k_frames<SRC, DST, KIND, WT>;
-        CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
-        FftTables tb{h->d_tw256, h->d_twsplit, h->d_twinv, h->d_win};
-        BatchDesc bd{p->d_pcm_off, p->d_nframes, p->d_row_off, ft.t32};
-        // from PCM: persistent CTAs, two per SM (shared-memory bound), each walks the tile list with stride
-        // gridDim.x and prefetches its next tile; other sources: one tile per CTA, the hardware scheduler overlaps them
-        int per_sm = 2;
-        if (SRC == SRC_PCM) CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, CTA_THREADS, bytes));
-        const unsigned grid = (SRC == SRC_PCM) ? (unsigned)std::min<int64_t>(ft.n32, std::max(per_sm, 1) * (int64_t)h->num_sms) : (unsigned)ft.n32;
-        h->lc.begin(names[SRC][DST], s);
-        kern<<<grid, CTA_THREADS, bytes, s>>>(P, bd, tb, pcm, src, dst, (int)ft.n32);
-        h->lc.end(s);
+        // 512-point band values and features come from the spectrum in k_bank (ctu_bank.cuh)
+        return fail(h, CTU_ERR_CONFIG, "CTU: internal: 512-point band values or features outside k_bank");
     }
-    CK(cudaGetLastError());
-    return CTU_OK;
 }
 
 template <int SRC, int DST, int KIND>
@@ -1150,7 +1120,7 @@ static int launch_frames_t(ctu_handle *h, const FrameParams &P, const ctu_plan *
                            const float *src, float *dst, cudaStream_t s) {
     // the PCM front end is specialised for the two standard window lengths (25 ms and 32 ms
     // at 16 kHz); every other length takes the generic instantiation
-    if constexpr (SRC == SRC_PCM) {
+    if constexpr (SRC == SRC_PCM && DST == DST_SPEC) {
         if (P.window == 400) return launch_frames_w<SRC, DST, KIND, 400>(h, P, p, ft, pcm, src, dst, s);
         if (P.window == 512) return launch_frames_w<SRC, DST, KIND, 512>(h, P, p, ft, pcm, src, dst, s);
     }
@@ -1287,7 +1257,7 @@ static int run_range(ctu_plan *p, const Range &r, const int16_t *d_pcm, const ui
     if (r.nrows <= 0 && !h->signal_out) return CTU_OK;
     BatchDesc bd32{p->d_pcm_off, p->d_nframes, p->d_row_off, p->d_tiles32 + r.t32_0};
     BatchDesc bd64{p->d_pcm_off, p->d_nframes, p->d_row_off, p->d_tiles64 + r.t64_0};
-    FrameTiles ft{p->d_tiles32 + r.t32_0, r.t32_n, p->d_tilesF + r.tF_0, r.tF_n};
+    FrameTiles ft{p->d_tilesF + r.tF_0, r.tF_n};
     int st;
     if (h->fea_kind == FEA_TDIIR)        // time-domain IIR filter bank -> band energies -> log -> DCT (ctu_tdiir.cuh)
         return launch_tdiir(h->tdp, bd64, r.t64_n, p->d_pcm_off, p->d_nframes, p->d_row_off, r.u0, r.u1, d_pcm, p->d_tdseg, d_fea, h->feature_dim, s,
@@ -1360,14 +1330,9 @@ static int run_range(ctu_plan *p, const Range &r, const int16_t *d_pcm, const ui
         CK(cudaGetLastError());
         return CTU_OK;
     }
-    if (h->signal_out && p->d_cspec) {
-        BatchDesc bdS{p->d_pcm_off, p->d_nframes, p->d_row_off, p->d_tilesS + r.tS_0};
-        return launch_synth_c(h->sp, h->fp, bdS, p->syn_tile, r.tS_n, p->d_osamp_off, p->d_cspec, p->d_spec, d_wave, h->d_tw256, h->d_twinv, s, &h->lc, h->err);
-    }
     if (h->signal_out) {
         BatchDesc bdS{p->d_pcm_off, p->d_nframes, p->d_row_off, p->d_tilesS + r.tS_0};
-        return launch_synth(h->sp, h->fp, bdS, p->syn_tile, r.tS_n, p->d_osamp_off, d_pcm, p->d_spec, d_wave, h->d_tw256, h->d_twsplit,
-                            h->d_twinv, h->d_win, s, &h->lc, h->err);
+        return launch_synth_c(h->sp, h->fp, bdS, p->syn_tile, r.tS_n, p->d_osamp_off, p->d_cspec, p->d_spec, d_wave, h->d_tw256, h->d_twinv, s, &h->lc, h->err);
     }
 
     // ---- stage 2: features ------------------------------------------------------------------
@@ -1812,7 +1777,6 @@ int ctu_set_option(ctu_handle *h, const char *name, int64_t value) {
     else if (n == "ss_carry") {
         // (re)starts a list: the buffer is zero before the first file of a reference process (Vec's constructor, src/base/types.h:35-38)
         if (value && h->nr_mode >= NR_HWSS) {
-            if (h->signal_out && h->synth_from_pcm) return fail(h, CTU_ERR_UNSUPPORTED, "CTU: ss_carry with synth_from_pcm (the sign of the Nyquist bin comes from the stored spectrum)");
             if (h->signal_out && h->bp.nfft) return fail(h, CTU_ERR_UNSUPPORTED, "CTU: ss_carry with waveform output at FFT sizes other than 512");
             CK(cudaSetDevice(h->device));
             const size_t nmax = (size_t)std::max(h->nbins, h->fb.nb) + 8;
@@ -1826,8 +1790,6 @@ int ctu_set_option(ctu_handle *h, const char *name, int64_t value) {
         }
         h->ss_carry = value != 0;
     }
-    else if (n == "split_front") h->split_front = value != 0;           // takes effect for plans created afterwards
-    else if (n == "synth_from_pcm") h->synth_from_pcm = value != 0;     // takes effect for plans created afterwards
     else if (n == "fuse_nr") h->fuse_nr = value != 0;
     else if (n == "front256") h->front256 = value != 0;                   // takes effect for plans created afterwards
     else return fail(h, CTU_ERR_CONFIG, "CTU: unknown run-time option " + n);
@@ -1854,7 +1816,7 @@ int ctu_debug_spectrum(ctu_plan *p, const int16_t *d_pcm, float *d_spec, void *s
     if (!p) return CTU_ERR_CONFIG;
     ctu_handle *h = p->h;
     CK(cudaSetDevice(h->device));
-    const FrameTiles ft{p->d_tiles32, p->tile32_off[p->n_utts], p->d_tilesF, p->tileF_off[p->n_utts]};
+    const FrameTiles ft{p->d_tilesF, p->tileF_off[p->n_utts]};
     FrameParams P = h->fp; P.out_dim = h->nbins; P.out_stride = h->nbins;
     // the kernels write rows of h->spitch floats (260 on the 512-point path); the tap hands out compact rows
     float *tmp = d_spec;

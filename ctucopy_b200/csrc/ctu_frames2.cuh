@@ -11,8 +11,8 @@
 // No [frames x 257] tile in shared memory: 38.9 KB per CTA; persistent CTAs, twiddles in registers, complex arithmetic on
 // packed FP32 instructions (ctu_fft.cuh).  Five resident CTAs (20 warps) per SM at 92 registers for 25 ms windows (window
 // values read from shared memory), four at up to 128 registers otherwise (window values in registers), against two CTAs
-// (16 warps) for the 32-frame tile kernel k_frames, which needs that tile for its lane = frame filter bank.  Measured on
-// 9.98 M frames: 6.0 ms here (first version: 7.3), 8.4 ms (persistent, prefetching) / 9.5 ms (plain) with k_frames.
+// (16 warps) for the 32-frame tile kernel k_frames it replaced, which needed that tile for its lane = frame filter bank.
+// Measured on 9.98 M frames: 6.0 ms here (first version: 7.3), 8.4 ms (persistent, prefetching) / 9.5 ms (plain) with k_frames.
 // Replaces rawIN::get_frame (src/io/in.cc:305-419).
 #ifndef CTU_FRAMES2_CUH
 #define CTU_FRAMES2_CUH

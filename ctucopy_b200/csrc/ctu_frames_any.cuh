@@ -1,5 +1,5 @@
 // K1g: the frame kernel for FFT sizes other than 512 (8 kHz telephone speech: 256 points;
-// 22-48 kHz audio: 1024 / 2048 points).  Same chain, same arithmetic conventions as k_frames
+// 22-48 kHz audio: 1024 / 2048 points).  Same chain, same arithmetic conventions as k_frames2 + k_bank
 // (rawIN::get_frame src/io/in.cc:305-419, FB::project_frame src/fea/fb.cc:72-86, specFEA /
 // logspecFEA / dctcFEA src/fea/fea_impl.cc:37-131), written for generality rather than speed:
 // one WARP per frame, the real transform as an in-place radix-2 complex FFT of half the length
@@ -120,7 +120,7 @@ k_frames_any(const __grid_constant__ FrameParams P, BatchDesc bd, AnyTables tb, 
         for (int i = threadIdx.x; i < P.nrows * nb; i += ANY_THREADS) d[(i % nb) * P.nrows + i / nb] = P.m2[(i / nb) * P.nbp + i % nb];
         m2t = d;
     }
-    if (tb.o_fbw >= 0 && SRC != SRC_FB && DST != DST_SPEC) { float *d = sm + tb.o_fbw; for (int i = threadIdx.x; i < tb.nfbw; i += ANY_THREADS) d[i] = tb.fbw[i]; fbwp = d; }
+    if (tb.o_fbw >= 0 && DST != DST_SPEC) { float *d = sm + tb.o_fbw; for (int i = threadIdx.x; i < tb.nfbw; i += ANY_THREADS) d[i] = tb.fbw[i]; fbwp = d; }
     __syncthreads();
     constexpr bool WANT_LOG = (DST == DST_FEA) && (KIND == KIND_DCTC || KIND == KIND_LOGSPEC || KIND == KIND_TRAPLOG);
     for (int f = wv; f < nf; f += ANY_THREADS / 32) {
@@ -223,12 +223,9 @@ k_frames_any(const __grid_constant__ FrameParams P, BatchDesc bd, AnyTables tb, 
                 if (k == 0 && P.remove_dc) p = 1e-10f;                // fixed floor (src/io/in.cc:390)
                 row[k] = P.take_sqrt ? sqrtf(p) : p;
             }
-        } else if (SRC == SRC_SPEC) {
+        } else {
             const float *g = src + (row0 + f) * nbins;
             for (int k = lane; k < nbins; k += 32) row[k] = g[k];
-        } else {
-            const float *g = src + (row0 + f) * nb;
-            for (int b = lane; b < nb; b += 32) { float v = g[b]; if (WANT_LOG) v = logf(v); sY[b] = v; }
         }
         __syncwarp();
         if (DST == DST_SPEC) {
@@ -237,28 +234,26 @@ k_frames_any(const __grid_constant__ FrameParams P, BatchDesc bd, AnyTables tb, 
             __syncwarp();
             continue;
         }
-        if (SRC != SRC_FB && (P.energy_mode == EN_NR || P.energy_mode == EN_IN)) {
+        if (P.energy_mode == EN_NR || P.energy_mode == EN_IN) {
             const float e = half_spectrum_energy(row, nbins, (P.energy_mode == EN_NR) || P.take_sqrt);
             if (lane == 0) P.energy[row0 + f] = e;
         }
         // ---- B: filter bank, one band per lane -----------------------------------------------------
         const bool late_log = (KIND == KIND_LOGSPEC && P.energy_mode == EN_BANDS && DST == DST_FEA);
-        if (SRC != SRC_FB) {
-            for (int b = lane; b < nb; b += 32) {
-                const int4 bs = __ldg(tb.bands + b);
-                const float *r = row + bs.x;
-                const float *wq = fbwp + bs.z;
-                float acc = 0.f;
-                for (int k = 0; k < bs.y; k++) acc = fmaf(r[k], wq[k], acc);   // the reference's summation order
-                const bool lg = WANT_LOG && !late_log;
-                float yv;
-                if (P.inld) { yv = powf(acc, 0.33f) * P.inld_scale; if (lg) yv = logf(yv); }
-                else yv = lg ? logf(acc) + P.log_offset : acc * P.lin_scale;
-                sY[b] = yv;
-            }
-            for (int b = nb + lane; b < P.nbp; b += 32) sY[b] = 0.f;
-            __syncwarp();
+        for (int b = lane; b < nb; b += 32) {
+            const int4 bs = __ldg(tb.bands + b);
+            const float *r = row + bs.x;
+            const float *wq = fbwp + bs.z;
+            float acc = 0.f;
+            for (int k = 0; k < bs.y; k++) acc = fmaf(r[k], wq[k], acc);   // the reference's summation order
+            const bool lg = WANT_LOG && !late_log;
+            float yv;
+            if (P.inld) { yv = powf(acc, 0.33f) * P.inld_scale; if (lg) yv = logf(yv); }
+            else yv = lg ? logf(acc) + P.log_offset : acc * P.lin_scale;
+            sY[b] = yv;
         }
+        for (int b = nb + lane; b < P.nbp; b += 32) sY[b] = 0.f;
+        __syncwarp();
         if (DST == DST_FB) {
             float *g = dst + (row0 + f) * nb;
             for (int b = lane; b < nb; b += 32) g[b] = sY[b];

@@ -220,9 +220,6 @@ int launch_burg(const BurgParams &B, int src_mode, const BatchDesc &bd, int64_t 
                 cudaStream_t s, LaunchCtx *lc, std::string &err);
 int launch_cepdet(const BurgParams &B, const int *d_nframes, const int64_t *d_row_off, int u0, int u1, const double *ceps,
                   uint8_t *flags, cudaStream_t s, LaunchCtx *lc, std::string &err);
-int launch_synth(const SynthParams &S, const FrameParams &F, const BatchDesc &bd, int tile_frames, int64_t ntiles,
-                 const int64_t *d_osamp_off, const int16_t *pcm, const float *spec, int16_t *out, const float2 *tw,
-                 const float2 *ts, const float2 *ti, const float *win, cudaStream_t s, LaunchCtx *lc, std::string &err);
 int launch_synth_c(const SynthParams &S, const FrameParams &F, const BatchDesc &bd, int tile_frames, int64_t ntiles,
                    const int64_t *d_osamp_off, const float2 *cspec, const float *spec, int16_t *out, const float2 *tw,
                    const float2 *ti, cudaStream_t s, LaunchCtx *lc, std::string &err);

@@ -251,9 +251,7 @@ int ctu_plan_fetch_vad_debug(ctu_plan *p, double *steps /* [total_frames x CTU_V
  *   "copy_only"      1 = the host entry points do their H2D / D2H copies with the kernels left out: the control
  *                        measurement behind bench.py's e2e.copy_only_ms
  *   "chunk_mb"       MB of PCM per pipeline chunk of the host entry points (default 32)
- *   "split_front"    1 (default) = PCM -> spectrum -> features as two kernels, 0 = the single fused frame kernel
- *   "synth_from_pcm" 1 = the synthesis recomputes the forward transform instead of reading the stored spectrum
- * The last two take effect for plans created afterwards.  Unknown name -> CTU_ERR_CONFIG.                          */
+ * Unknown name -> CTU_ERR_CONFIG.                                                                                  */
 int ctu_set_option(ctu_handle *h, const char *name, int64_t value);
 
 /* Page-locked host memory for the buffers handed to ctu_plan_run_host / ctu_run: pageable memory

@@ -183,12 +183,9 @@ def test_cuda_matches_oracle_on_parity_set(name):
             assert np.array_equal(got.astype(bool), ref.vad_nr), (name, j, "detector decisions differ at %d frames" % int((got.astype(bool) != ref.vad_nr).sum()))
 
 
-# every alternative kernel path of the BASELINE configurations (run-time options, ctu_set_option): the fused frame kernel
-# instead of PCM -> spectrum -> k_bank, the standalone scan instead of the one fused into k_bank, and the synthesis that
-# recomputes the forward transform instead of reading the stored spectrum
-ALT_PATHS = [("mfcc_d_a", {"split_front": 0}), ("plp", {"split_front": 0}), ("trapdct", {"split_front": 0}),
-             ("mfcc_exten", {"fuse_nr": 0}), ("mfcc_exten", {"fuse_nr": 1}), ("fwss_burg", {"fuse_nr": 0}), ("fwss_burg", {"fuse_nr": 1}),
-             ("exten_raw", {"synth_from_pcm": 1})]
+# every alternative kernel path of the BASELINE configurations (run-time options, ctu_set_option): the standalone scan
+# instead of the one fused into k_bank
+ALT_PATHS = [("mfcc_exten", {"fuse_nr": 0}), ("mfcc_exten", {"fuse_nr": 1}), ("fwss_burg", {"fuse_nr": 0}), ("fwss_burg", {"fuse_nr": 1})]
 
 
 @pytest.mark.parametrize("name,options", ALT_PATHS, ids=["%s-%s" % (n, "+".join("%s=%d" % kv for kv in o.items())) for n, o in ALT_PATHS])
