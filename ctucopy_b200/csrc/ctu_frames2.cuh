@@ -3,16 +3,17 @@
 //
 // A CTA of 128 threads = 8 groups of 16 threads works on a tile of 16 consecutive frames of
 // one utterance.  The CTA synchronises once, after staging the tile's pre-emphasised samples
-// and the (small) tables in shared memory; from then on each group takes a frame through
+// (four per thread, finish_pcm) and the (small) tables in shared memory; the descriptors of
+// the next tiles arrive ahead in shared memory (TileAhead); from then on each group takes a frame through
 //   window, DC removal -> 256-point complex FFT (16 points per thread, ctu_fft.cuh) -> real
 //   split by register shuffles -> power / magnitude
 // on its own, synchronising only inside its half warp, and stores its 257 bins from the
 // registers straight to HBM (every store instruction covers 64 contiguous bytes).
-// No [frames x 257] tile in shared memory: 38.9 KB per CTA; persistent CTAs, twiddles in registers, complex arithmetic on
-// packed FP32 instructions (ctu_fft.cuh).  Five resident CTAs (20 warps) per SM at 92 registers for 25 ms windows (window
+// No [frames x 257] tile in shared memory: 39.0 KB per CTA; persistent CTAs, twiddles in registers, complex arithmetic on
+// packed FP32 instructions (ctu_fft.cuh).  Five resident CTAs (20 warps) per SM at 94 registers for 25 ms windows (window
 // values read from shared memory), four at up to 128 registers otherwise (window values in registers), against two CTAs
 // (16 warps) for the 32-frame tile kernel k_frames it replaced, which needed that tile for its lane = frame filter bank.
-// Measured on 9.98 M frames: 6.0 ms here (first version: 7.3), 8.4 ms (persistent, prefetching) / 9.5 ms (plain) with k_frames.
+// Measured on 9.98 M frames: 5.63 ms here (first version: 7.3), 8.4 ms (persistent, prefetching) / 9.5 ms (plain) with k_frames.
 // Replaces rawIN::get_frame (src/io/in.cc:305-419).
 #ifndef CTU_FRAMES2_CUH
 #define CTU_FRAMES2_CUH
@@ -27,7 +28,7 @@ constexpr int F2_TILE = 16;                     // frames per CTA: two passes
 constexpr int F2_ROWF = 2 * XPAD * 16;          // floats in a group's exchange area (544)
 
 struct Smem2 {
-    int oX, oTw, oTs, oW, oD, oRaw, total;      // float offsets
+    int oX, oTw, oTs, oW, oD, oRaw, oA, total;  // float offsets
 };
 __host__ __device__ inline Smem2 smem2_layout(int window, int wshift) {
     Smem2 L;
@@ -38,6 +39,7 @@ __host__ __device__ inline Smem2 smem2_layout(int window, int wshift) {
     L.oW = o; o += (window + 3) & ~3;
     L.oD = o; o += ((F2_TILE - 1) * wshift + window + 7) & ~7;
     L.oRaw = o; o += (((F2_TILE - 1) * wshift + window + 1 + 8 + 7) / 8) * 4;   // int16 prefetch buffer: 8-sample chunks
+    L.oA = o; o += TILE_AHEAD_FLOATS;
     L.total = o;
     return L;
 }
@@ -47,8 +49,9 @@ __host__ __device__ inline Smem2 smem2_layout(int window, int wshift) {
 // WSM: the thread's 32 window values come from shared memory (16 eight-byte loads per frame) instead of living in
 // registers.  With packed arithmetic the kernel is latency bound at four CTAs per SM (ncu: issue slots 54 %, FP32 pipe 29 %,
 // shared-memory wavefronts 61 %, 16 warps per SM); without the 32 registers the 25 ms window fits five CTAs (92 registers,
-// no spills): 6.19 -> 6.05 ms per 9.98 M frames (tools/gpu_jobs/r2_job46.sh).  The other instantiations would spill at 102
-// registers (32 ms window, stored complex spectrum: 5.80 -> 6.33 ms) and keep the window in registers at four CTAs.
+// no spills; 94 since the descriptor and staging changes): 6.19 -> 6.05 ms per 9.98 M frames (tools/gpu_jobs/r2_job46.sh).
+// The other instantiations would spill at 102 registers (32 ms window, stored complex spectrum: 5.80 -> 6.33 ms) and keep
+// the window in registers at four CTAs.
 template <int WT, bool CPLX> struct F2Cfg {
     static constexpr bool wsm = (WT == 400) && !CPLX;
     static constexpr int minb = wsm ? 5 : 4;
@@ -69,6 +72,8 @@ k_frames2(const __grid_constant__ FrameParams P, BatchDesc bd, FftTables tb, con
     int tile = blockIdx.x;
     if (tile >= ntiles) return;
     TileMeta cur = load_tile_meta(bd, tile, s, F2_TILE);
+    TileAhead *ahead = reinterpret_cast<TileAhead *>(sm + L.oA);
+    tile_ahead_init(ahead, bd, tile, ntiles);
     int edge = 0;
     prefetch_pcm<F2_THREADS>(raw, pcm, cur, (cur.nf - 1) * s + w + 1, edge);
     for (int i = tid; i < w; i += F2_THREADS) sW[i] = tb.win[i];
@@ -100,14 +105,13 @@ k_frames2(const __grid_constant__ FrameParams P, BatchDesc bd, FftTables tb, con
     twr[3] = sTw[64 + c]; twr[4] = sTw[128 + c]; twr[5] = sTw[192 + c];
     const cpx<float> ts_c = sTs[c];
 #pragma unroll 1
-    for (; tile < ntiles; tile += gridDim.x) {
+    for (int j = 0; tile < ntiles; tile += gridDim.x, j ^= 1) {
     const int next = tile + gridDim.x;
-    TileMeta nxt = cur;
-    if (next < ntiles) nxt = load_tile_meta(bd, next, s, F2_TILE);
     const int nf = cur.nf;
     const int64_t row0 = cur.row0;
     finish_pcm<F2_THREADS>(raw, sD, pcm, cur, (nf - 1) * s + w + 1, edge, P.preem);
     __syncthreads();                                          // samples staged; the raw buffer is free again
+    const TileMeta nxt = tile_ahead_next(ahead, j, bd, tile, ntiles, s, F2_TILE);   // used only when next < ntiles
     if (next < ntiles) prefetch_pcm<F2_THREADS>(raw, pcm, nxt, (nxt.nf - 1) * s + w + 1, edge);
     // the two groups of a warp walk the tile in step (frames grp, grp + 8): with an odd number of frames the last group
     // recomputes the tile's last frame and stores nothing -- every shuffle can then name the full warp (bare SHFL)

@@ -39,7 +39,8 @@ struct Tables256 {
 __host__ __device__ inline int smem256_samples(int window, int wshift) { return ((F256_TILE - 1) * wshift + window + 7) & ~7; }
 __host__ __device__ inline int smem256_raw(int window, int wshift) { return (((F256_TILE - 1) * wshift + window + 1 + 8 + 7) / 8) * 4; }
 __host__ __device__ inline size_t smem256_floats(int window, int wshift) {
-    return (size_t)2 * F256_TILE * F256_GRP + 2 * 128 + 2 * 130 + 256 + smem256_samples(window, wshift) + smem256_raw(window, wshift);
+    return (size_t)2 * F256_TILE * F256_GRP + 2 * 128 + 2 * 130 + 256 + smem256_samples(window, wshift) + smem256_raw(window, wshift) +
+           TILE_AHEAD_FLOATS;
 }
 
 // (dft8 and the index algebra of the 16 x 8 decomposition: ctu_fft.cuh, emulated on the CPU by tests/emu/emu_fft.cpp)
@@ -50,7 +51,8 @@ __device__ __forceinline__ float group_sum8(float v) {
     return v;
 }
 
-__global__ void __launch_bounds__(F256_THREADS)
+// five resident CTAs per SM (at most 96 registers, no spills); left to itself ptxas takes 117 registers, which leaves four
+__global__ void __launch_bounds__(F256_THREADS, 5)
 k_frames256(const __grid_constant__ FrameParams P, BatchDesc bd, Tables256 tb, const int16_t *__restrict__ pcm, float *__restrict__ dst, int nbins,
             int ntiles) {
     extern __shared__ __align__(16) float sm[];
@@ -62,10 +64,12 @@ k_frames256(const __grid_constant__ FrameParams P, BatchDesc bd, Tables256 tb, c
     float *sW = reinterpret_cast<float *>(sTs + 130);                                   // 256
     float *sD = sW + 256;                                                               // the tile's pre-emphasised samples
     int16_t *raw = reinterpret_cast<int16_t *>(sD + smem256_samples(w, s));             // int16 prefetch buffer
+    TileAhead *ahead = reinterpret_cast<TileAhead *>(sD + smem256_samples(w, s) + smem256_raw(w, s));
     // persistent CTAs: the next tile's PCM travels HBM -> shared memory (cp.async) while this one is transformed
     int tile = blockIdx.x;
     if (tile >= ntiles) return;
     TileMeta cur = load_tile_meta(bd, tile, s, F256_TILE);
+    tile_ahead_init(ahead, bd, tile, ntiles);
     int edge = 0;
     prefetch_pcm<F256_THREADS>(raw, pcm, cur, (cur.nf - 1) * s + w + 1, edge);
     for (int i = tid; i < 128; i += F256_THREADS) sTw[i] = mk<float>(tb.tw128[i].x, tb.tw128[i].y);
@@ -73,13 +77,12 @@ k_frames256(const __grid_constant__ FrameParams P, BatchDesc bd, Tables256 tb, c
     for (int i = tid; i < 256; i += F256_THREADS) sW[i] = (i < w) ? tb.win[i] : 0.f;
     cpx<float> *xch = sX + grp * F256_GRP;
 #pragma unroll 1
-    for (; tile < ntiles; tile += gridDim.x) {
+    for (int j = 0; tile < ntiles; tile += gridDim.x, j ^= 1) {
     const int next = tile + gridDim.x;
-    TileMeta nxt = cur;
-    if (next < ntiles) nxt = load_tile_meta(bd, next, s, F256_TILE);
     const int nf = cur.nf;
     finish_pcm<F256_THREADS>(raw, sD, pcm, cur, (nf - 1) * s + w + 1, edge, P.preem);   // pre-emphasis once per sample
     __syncthreads();                                       // samples (and, the first time, the tables) staged; raw is free again
+    const TileMeta nxt = tile_ahead_next(ahead, j, bd, tile, ntiles, s, F256_TILE);   // used only when next < ntiles
     if (next < ntiles) prefetch_pcm<F256_THREADS>(raw, pcm, nxt, (nxt.nf - 1) * s + w + 1, edge);
     // a group past the end of the tile recomputes the tile's last frame and stores nothing (shuffles name the full warp)
     const bool store = grp < nf;

@@ -166,21 +166,92 @@ __device__ __forceinline__ float half_spectrum_energy(const float *row, int n, b
 
 // int16 -> float without the (quarter-rate) conversion pipe: 1.5*2^23 + x is exact
 __device__ __forceinline__ float s16_to_f32(int x) { return __int_as_float(0x4B400000 + x) - 12582912.0f; }
+// two int16 (a little-endian pair: element 2j in the low half) -> two floats, exactly: with the sign bits flipped the halves are
+// v + 32768 in 0..65535, which PRMT places under the exponent of 2^23 (no sign extension); one packed subtraction of
+// 2^23 + 2^15 leaves v
+__device__ __forceinline__ cpx<float> s16x2_to_f32x2(uint32_t p) {
+    const uint32_t q = p ^ 0x80008000u;
+    const cpx<float> b = mk<float>(__uint_as_float(__byte_perm(q, 0x4B000000u, 0x7610)), __uint_as_float(__byte_perm(q, 0x4B000000u, 0x7632)));
+    return b - mk<float>(8421376.0f, 8421376.0f);
+}
 
 // ---- PCM prefetch: the next tile's samples travel HBM -> shared memory with cp.async while the
 // current tile is being transformed (the CTAs are persistent).  The raw int16 buffer keeps the
 // 16-byte phase of the source address so that whole 16-byte chunks can be copied; the (at most
 // two) partial chunks at the ends go through a register.
-struct TileMeta { int u, t0, nf; int64_t row0, g0; };
+struct TileMeta { int t0, nf; int64_t row0, g0; };
 
-__device__ __forceinline__ TileMeta load_tile_meta(const BatchDesc &bd, int tile, int wshift, int tile_frames = TILE_F) {
+// a tile's list entry resolved against its utterance, as loaded; tile_meta turns it into the TileMeta
+struct TileDesc { int t0, nfu; int64_t roff, poff; };
+
+__device__ __forceinline__ TileDesc load_tile_desc(const BatchDesc &bd, int2 t) {
+    TileDesc d;
+    d.t0 = t.y;
+    d.nfu = bd.nframes[t.x];
+    d.roff = bd.row_off[t.x];
+    d.poff = bd.pcm_off[t.x];
+    return d;
+}
+
+__device__ __forceinline__ TileMeta tile_meta(const TileDesc &d, int wshift, int tile_frames) {
     TileMeta m;
-    const int2 t = bd.tiles[tile];
-    m.u = t.x; m.t0 = t.y;
-    m.nf = min(tile_frames, bd.nframes[m.u] - m.t0);
-    m.row0 = bd.row_off[m.u] + m.t0;
-    m.g0 = bd.pcm_off[m.u] + (int64_t)m.t0 * wshift;
+    m.t0 = d.t0;
+    m.nf = min(tile_frames, d.nfu - d.t0);
+    m.row0 = d.roff + d.t0;
+    m.g0 = d.poff + (int64_t)d.t0 * wshift;
     return m;
+}
+
+__device__ __forceinline__ TileMeta load_tile_meta(const BatchDesc &bd, int tile, int wshift, int tile_frames) {
+    return tile_meta(load_tile_desc(bd, bd.tiles[tile]), wshift, tile_frames);
+}
+
+// Descriptors of the tiles a persistent CTA takes next (tile + G, tile + 2G, ...; G = gridDim.x), fetched ahead by thread 0
+// with cp.async into shared memory: in the iteration of `tile`, the per-utterance values of tile + 2G and the list entry of
+// tile + 3G.  They land by the cp.async wait of the next iteration, so no load is consumed in the iteration that issues it.
+// (The values are warp uniform, and the compiler moves a loaded one into a uniform register as soon as its load returns:
+// with global loads the whole CTA waited there for two dependent load latencies per tile, and holding the values in
+// ordinary registers across the transform costs the registers of the fifth CTA.)  Two slots, alternating by iteration.
+struct TileAhead {
+    int64_t roff[2], poff[2];
+    int2 t[2];
+    int nfu[2], t0[2];
+};
+constexpr int TILE_AHEAD_FLOATS = (int)(sizeof(TileAhead) / 4);   // 16: a multiple of four keeps what follows 16-byte aligned
+
+__device__ __forceinline__ void cp_async_small(void *dst, const void *src, int bytes) {
+    const unsigned d = (unsigned)__cvta_generic_to_shared(dst);
+    if (bytes == 8) asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(d), "l"(src) : "memory");
+    else asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(d), "l"(src) : "memory");
+}
+
+// thread 0: the per-utterance values of list entry e into slot j
+__device__ __forceinline__ void tile_ahead_desc(TileAhead *A, int j, const BatchDesc &bd, int2 e) {
+    A->t0[j] = e.y;
+    cp_async_small(&A->nfu[j], bd.nframes + e.x, 4);
+    cp_async_small(&A->roff[j], bd.row_off + e.x, 8);
+    cp_async_small(&A->poff[j], bd.pcm_off + e.x, 8);
+}
+
+// before the first tile (the copies join the first PCM prefetch's group)
+__device__ __forceinline__ void tile_ahead_init(TileAhead *A, const BatchDesc &bd, int tile, int ntiles) {
+    const int G = gridDim.x;
+    if (threadIdx.x != 0) return;
+    if (tile + G < ntiles) tile_ahead_desc(A, 0, bd, bd.tiles[tile + G]);
+    if (tile + 2 * G < ntiles) cp_async_small(&A->t[0], bd.tiles + tile + 2 * G, 8);
+}
+
+// in the iteration of `tile` (slot j = its parity), after the cp.async wait and a barrier: the descriptor of tile + G
+// (meaningful when tile + G < ntiles); thread 0 then issues the copies that the next iteration reads from slot j ^ 1
+__device__ __forceinline__ TileMeta tile_ahead_next(TileAhead *A, int j, const BatchDesc &bd, int tile, int ntiles, int wshift,
+                                                    int tile_frames) {
+    const TileDesc d = TileDesc{A->t0[j], A->nfu[j], A->roff[j], A->poff[j]};
+    if (threadIdx.x == 0) {
+        const int G = gridDim.x;
+        if (tile + 2 * G < ntiles) tile_ahead_desc(A, j ^ 1, bd, A->t[j]);
+        if (tile + 3 * G < ntiles) cp_async_small(&A->t[j ^ 1], bd.tiles + tile + 3 * G, 8);
+    }
+    return tile_meta(d, wshift, tile_frames);
 }
 
 // element k of the tile's sample run is sample (k - 1): k = 0 is the sample before the tile
@@ -229,9 +300,28 @@ __device__ __forceinline__ void finish_pcm(int16_t *raw, float *__restrict__ sD,
     __syncthreads();
     const int16_t *x = raw + phase;                       // x[k]: element k
     const int nsamp = n - 1;
-    // consecutive threads take consecutive samples: 2-byte reads and 4-byte writes at unit stride are free of bank
-    // conflicts (the 8-samples-per-thread layout cost four wavefronts per load: ncu, profiles/)
-    for (int i = threadIdx.x; i < nsamp; i += NT) {
+    int i0 = 0;
+    if (phase & 1) {
+        // x + 1 is 4-byte aligned: a thread takes four consecutive samples -- two int16 pairs, the sample before them and
+        // one 16-byte store.  Consecutive threads take consecutive runs, so a warp's pair loads cover 256 contiguous bytes
+        // (two wavefronts each), the loads of the sample before (stride 8 bytes) two, and its store 512 contiguous bytes
+        // (four): 10 wavefronts per 128 samples against 12 for four rounds of the scalar loop below, in a quarter of the
+        // loop iterations.  (An earlier 8-samples-per-thread layout lost to the scalar loop: it cost four wavefronts per
+        // load; ncu, profiles/.  Here no access spans more bytes than it moves.)
+        const int nq = nsamp >> 2;
+#pragma unroll 2   // fully unrolled, the loop costs the 32-register-window instantiations of k_frames2 a spill
+        for (int q = threadIdx.x; q < nq; q += NT) {
+            const int i = 4 * q;
+            const uint32_t *xp = reinterpret_cast<const uint32_t *>(x + i + 1);
+            const cpx<float> a = s16x2_to_f32x2(xp[0]), b = s16x2_to_f32x2(xp[1]);
+            const float p = s16_to_f32((int)x[i]);
+            *reinterpret_cast<float4 *>(sD + i) =
+                make_float4(fmaf(-alpha, p, a.x), fmaf(-alpha, a.x, a.y), fmaf(-alpha, a.y, b.x), fmaf(-alpha, b.x, b.y));
+        }
+        i0 = 4 * nq;
+    }
+    // even phases (odd utterance offsets or shifts), and the last nsamp % 4 samples of odd ones: one sample per thread
+    for (int i = i0 + threadIdx.x; i < nsamp; i += NT) {
         const float prev = s16_to_f32((int)x[i]);
         const float xi = s16_to_f32((int)x[i + 1]);
         sD[i] = fmaf(-alpha, prev, xi);
