@@ -67,16 +67,25 @@ __device__ __forceinline__ void warp_fft_radix2(cpx<double> *z, int M, int log2m
 }
 
 // the frame exactly as rawIN::get_frame builds it (pre-emphasis, window, mean of the windowed frame removed inside the
-// window, src/io/in.cc:362-388), transformed: z holds FFT_M of the even/odd packed frame afterwards
+// window, src/io/in.cc:362-388), transformed: z holds FFT_M of the even/odd packed frame afterwards.
+// DC1 (-remove_dc1): the samples are first taken as the de-meaned ring holds them at frame t of the utterance; m points at
+// that frame's ring mean (k_dc1_means), s is the shift.
+template <bool DC1 = false>
 __device__ __forceinline__ void any64_analysis(cpx<double> *z, const AnyTables64 &tb, const int16_t *__restrict__ x, bool at_start, int w,
-                                               double preem, int remove_dc, int lane) {
+                                               double preem, int remove_dc, int lane, const double *__restrict__ m = nullptr, int t = 0,
+                                               int s = 0) {
     const int nfft = tb.nfft;
     double sum = 0.0;
     for (int i = lane; i < nfft; i += 32) {
         double v = 0.0;
         if (i < w) {
-            const double xi = (double)x[i];
-            const double xp = (i == 0 && at_start) ? 0.0 : (double)x[i - 1];
+            double xi = (double)x[i];
+            double xp = (i == 0 && at_start) ? 0.0 : (double)x[i - 1];
+            if (DC1) {
+                xi = dc1_ring_value(xi, m, i, 0, t, w, s);
+                if (i > 0) xp = dc1_ring_value(xp, m, i - 1, 0, t, w, s);
+                else if (!at_start) xp = dc1_ring_value(xp, m, s - 1, 1, t, w, s);
+            }
             v = tb.win[i] * (xi - preem * xp);
         }
         any64_real(z, i) = v;

@@ -642,7 +642,7 @@ static int resolve_modes(ctu_handle *h) {
             return fail(h, CTU_ERR_UNSUPPORTED, "CTU: -fea_Z_exp is built for cepstral features (dctc, lpc) and for delta / stacking chains");
         if (h->do_vad) return fail(h, CTU_ERR_UNSUPPORTED, "CTU: -fea_Z_exp together with the VAD module");
     }
-    // -remove_dc1 needs per-frame ring offsets: only the general kernel applies them
+    // -remove_dc1 needs per-frame ring offsets: only the general kernels apply them
     // dither (src/io/in.cc:452-455): glibc's rand() stream restated on the host, one value per loaded sample in list
     // order; applied by the general kernel
     h->generic = !h->fea_in && ((c.wfft != NFFT) || c.remove_dc1 || c.dither != 0.0);
@@ -652,15 +652,14 @@ static int resolve_modes(ctu_handle *h) {
     h->nbins = c.wfftby2;
     h->spitch = h->generic ? h->nbins : SPITCH;      // 512-point path: rows padded to 260 floats (16-byte aligned)
     if (c.remove_dc1 && c.window / c.wshift + 1 > ANY_DC1_MAX) return fail(h, CTU_ERR_UNSUPPORTED, "CTU: -remove_dc1 with a window longer than 17 shifts");
-    if (c.remove_dc1 && c.fea_E && c.fea_rawenergy) return fail(h, CTU_ERR_UNSUPPORTED, "CTU: -remove_dc1 together with -fea_rawenergy");
     if (h->generic) {
         // other sampling rates / window lengths, -remove_dc1, -dither: the general (slower) frame kernel; synthesis, the Burg
-        // detector and the fp64 path have general siblings too (ctu_any64.cuh), but those do not apply ring offsets / dither
+        // detector and the fp64 path have general siblings too (ctu_any64.cuh), which apply the ring offsets of -remove_dc1
+        // but not the noise of -dither
         if (c.wfft < 64 || c.wfft > ANY_MAX_NFFT) return fail(h, CTU_ERR_UNSUPPORTED, "CTU: FFT sizes from 64 to 2048 points are built (window of 33..2048 samples)");
-        if (h->signal_out && (c.remove_dc1 || c.dither != 0.0))
-            return fail(h, CTU_ERR_UNSUPPORTED, "CTU: waveform output together with -remove_dc1 / -dither");
-        if ((h->vad_src == VADSRC_BURG || (h->do_vad && h->vad_cri == VCRI_CEPDIST_LPC)) && (c.remove_dc1 || c.dither != 0.0))
-            return fail(h, CTU_ERR_UNSUPPORTED, "CTU: the Burg detector together with -remove_dc1 / -dither");
+        if (h->signal_out && c.dither != 0.0) return fail(h, CTU_ERR_UNSUPPORTED, "CTU: waveform output together with -dither");
+        if ((h->vad_src == VADSRC_BURG || (h->do_vad && h->vad_cri == VCRI_CEPDIST_LPC)) && c.dither != 0.0)
+            return fail(h, CTU_ERR_UNSUPPORTED, "CTU: the Burg detector together with -dither");
     }
     return CTU_OK;
 }
@@ -776,11 +775,14 @@ int ctu_create(const ctu_config *cfg, int device, ctu_handle **out) {
     // decisions must match the reference bit for bit: features in fp64 like the reference's
     if (h->do_vad && h->vad_cri == VCRI_CEPDIST_FEA) h->precise = true;
     // the fp64 general kernels (ctu_any64.cuh) also take the 512-point frames whose window length is odd (e.g. 32 ms at
-    // 11.025 kHz = 353 samples): the specialised synthesis / Burg kernels pair samples two by two
-    const bool any64 = c_wfft_is_general(h) || (h->cfg.window & 1);
+    // 11.025 kHz = 353 samples): the specialised synthesis / Burg kernels pair samples two by two.  They take -remove_dc1
+    // at every size too: k_synth_c and k_burg read X from k_frames2, which applies no ring offsets, and k_frames_any
+    // (the spectrum under -remove_dc1) does not store X.  The spectrum that feeds the noise reduction and the features
+    // stays on k_frames_any.
+    const bool any64 = c_wfft_is_general(h) || (h->cfg.window & 1) || h->cfg.remove_dc1;
     if (h->generic || any64) {
-        if (h->generic && h->precise && (h->cfg.remove_dc1 || h->cfg.dither != 0.0)) {
-            h->err = "CTU: -remove_dc1 / -dither together with a configuration that needs the fp64 path (band-domain noise reduction, LPC without the cube-root law, feature-vector VAD)";
+        if (h->generic && h->precise && h->cfg.dither != 0.0) {
+            h->err = "CTU: -dither together with a configuration that needs the fp64 path (band-domain noise reduction, LPC without the cube-root law, feature-vector VAD)";
             return bail(CTU_ERR_UNSUPPORTED);
         }
         const int N = h->cfg.wfft, M = N / 2;
@@ -1270,6 +1272,8 @@ static int run_range(ctu_plan *p, const Range &r, const int16_t *d_pcm, const ui
     const bool before = h->cfg.nr_when == 0 || h->signal_out;
     const bool need_spec = p->d_spec != nullptr;
     FrameParams P = h->fp;
+    BurgParams BP = h->bp;
+    BP.dc1 = p->d_dc1;
     if (p->d_dc1 && r.u1 > r.u0) {
         h->lc.begin("k_dc1_means", s);
         k_dc1_means<<<(unsigned)((r.u1 - r.u0 + 3) / 4), 128, 0, s>>>(p->d_nframes, p->d_row_off, p->d_pcm_off, r.u0, r.u1 - r.u0, h->cfg.window,
@@ -1292,7 +1296,7 @@ static int run_range(ctu_plan *p, const Range &r, const int16_t *d_pcm, const ui
     const bool fuse_scan = bank_path && nr_on && before && h->fuse_nr && !h->do_vad && h->nrp.a_kind != 0 && !carry;
     if (nr_on && before) {
         if (h->nr_mode >= NR_HWSS && h->vad_src == VADSRC_BURG) {
-            if ((st = launch_burg(h->bp, BURG_SRC_NR, bd32, r.t32_n, d_pcm, nullptr, p->d_ceps, h->d_tw256d, h->d_twsplitd, h->d_twinvd, h->d_wind,
+            if ((st = launch_burg(BP, BURG_SRC_NR, bd32, r.t32_n, d_pcm, nullptr, p->d_ceps, h->d_tw256d, h->d_twsplitd, h->d_twinvd, h->d_wind,
                                   h->d_hann, s, &h->lc, h->err))) return st;
             if ((st = launch_cepdet(h->bp, p->d_nframes, p->d_row_off, r.u0, r.u1, p->d_ceps, flags, s, &h->lc, h->err))) return st;
         }
@@ -1318,10 +1322,11 @@ static int run_range(ctu_plan *p, const Range &r, const int16_t *d_pcm, const ui
         while ((1 << lg) < M) lg++;
         AnyTables64 tb{h->d_any_tw64, h->d_any_ts64, h->d_wind, N, lg, h->spitch};
         const size_t bytes = (size_t)(SYNANY_THREADS / 32) * (2 * any64_zslots(M) + 2 * (M + 2)) * sizeof(double);
-        CK(cudaFuncSetAttribute(k_synth_frames_any, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
+        auto ks = p->d_dc1 ? k_synth_frames_any<true> : k_synth_frames_any<false>;
+        CK(cudaFuncSetAttribute(ks, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
         h->lc.begin("k_synth_frames_any", s);
-        k_synth_frames_any<<<(unsigned)r.tF_n, SYNANY_THREADS, bytes, s>>>(h->cfg.window, h->cfg.wshift, (double)h->cfg.preem, h->cfg.remove_dc, bdF, tb, d_pcm,
-                                                                          p->d_spec, p->d_yt);
+        ks<<<(unsigned)r.tF_n, SYNANY_THREADS, bytes, s>>>(h->cfg.window, h->cfg.wshift, (double)h->cfg.preem, h->cfg.remove_dc, bdF, tb, d_pcm, p->d_spec, p->d_yt,
+                                                          p->d_dc1);
         h->lc.end(s);
         CK(cudaGetLastError());
         h->lc.begin("k_ola_any", s);
@@ -1403,7 +1408,8 @@ static int run_range(ctu_plan *p, const Range &r, const int16_t *d_pcm, const ui
     if (h->energy_mode && r.t64_n > 0) {
         if (h->energy_mode == EN_RAW) {
             h->lc.begin("k_rawenergy", s);
-            k_rawenergy<<<(unsigned)r.t64_n, 256, 0, s>>>(bd64, h->cfg.window, h->cfg.wshift, d_pcm, p->d_E);
+            if (p->d_dc1) k_rawenergy<true><<<(unsigned)r.t64_n, 256, 0, s>>>(bd64, h->cfg.window, h->cfg.wshift, d_pcm, p->d_E, p->d_dc1);
+            else k_rawenergy<false><<<(unsigned)r.t64_n, 256, 0, s>>>(bd64, h->cfg.window, h->cfg.wshift, d_pcm, p->d_E, nullptr);
             h->lc.end(s);
         }
         h->lc.begin("k_place_energy", s);
@@ -1415,7 +1421,7 @@ static int run_range(ctu_plan *p, const Range &r, const int16_t *d_pcm, const ui
     if (h->do_vad) {
         VadParams VP = h->vp;
         VP.dbg = p->d_vdbg;
-        if ((st = launch_vad_module(VP, h->bp, bd32, r.t32_n, p->d_nframes, p->d_row_off, r.u0, r.u1, r.row0, r.nrows, d_pcm, p->d_spec, d_fea,
+        if ((st = launch_vad_module(VP, BP, bd32, r.t32_n, p->d_nframes, p->d_row_off, r.u0, r.u1, r.row0, r.nrows, d_pcm, p->d_spec, d_fea,
                                     p->d_fea64, h->feature_dim, p->d_ceps, p->d_cri, p->d_vad0, d_vadout, p->d_keep, p->d_rows, h->d_tw256d, h->d_twsplitd,
                                     h->d_twinvd, h->d_wind, s, &h->lc, h->err))) return st;
     }
@@ -1777,7 +1783,8 @@ int ctu_set_option(ctu_handle *h, const char *name, int64_t value) {
     else if (n == "ss_carry") {
         // (re)starts a list: the buffer is zero before the first file of a reference process (Vec's constructor, src/base/types.h:35-38)
         if (value && h->nr_mode >= NR_HWSS) {
-            if (h->signal_out && h->bp.nfft) return fail(h, CTU_ERR_UNSUPPORTED, "CTU: ss_carry with waveform output at FFT sizes other than 512");
+            if (h->signal_out && h->bp.nfft)
+                return fail(h, CTU_ERR_UNSUPPORTED, "CTU: ss_carry with waveform output on the general synthesis (FFT sizes other than 512, odd window lengths, -remove_dc1)");
             CK(cudaSetDevice(h->device));
             const size_t nmax = (size_t)std::max(h->nbins, h->fb.nb) + 8;
             if (!h->d_carry) CK(cudaMalloc(&h->d_carry, nmax * sizeof(float)));

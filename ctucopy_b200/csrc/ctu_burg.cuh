@@ -354,6 +354,8 @@ k_burg(const __grid_constant__ BurgParams B, int src_mode, BatchDesc bd, int nha
 // doubles of shared memory per warp of k_burg_any: z (padded), Y, eb
 __host__ __device__ inline size_t burg_any_doubles(int M) { return (size_t)2 * any64_zslots(M) + 2 * (M + 2) + 2 * M; }
 
+// DC1: -remove_dc1, the frame is built from the de-meaned ring (B.dc1)
+template <bool DC1>
 __global__ void __launch_bounds__(ANY64_THREADS)
 k_burg_any(const __grid_constant__ BurgParams B, int src_mode, BatchDesc bd, AnyTables64 tb, const int16_t *__restrict__ pcm,
            const float *__restrict__ spec, double *__restrict__ ceps, const double *__restrict__ g_hann) {
@@ -371,7 +373,7 @@ k_burg_any(const __grid_constant__ BurgParams B, int src_mode, BatchDesc bd, Any
     const int w = B.window, s = B.wshift;
     const int ncoef = (src_mode == BURG_SRC_NR) ? B.ncoef_nr : B.ncoef_vad;
     for (int f = wv; f < nf; f += ANY64_THREADS / 32) {
-        any64_analysis(z, tb, pcm + bd.pcm_off[u] + (int64_t)(t0 + f) * s, (t0 + f) == 0, w, B.preem, B.remove_dc, lane);
+        any64_analysis<DC1>(z, tb, pcm + bd.pcm_off[u] + (int64_t)(t0 + f) * s, (t0 + f) == 0, w, B.preem, B.remove_dc, lane, DC1 ? B.dc1 + row0 + f : nullptr, t0 + f, s);
         // (|X|^a or the post-NR spectrum) with the phase of X -- see k_burg for the conventions (bin 0: phase 0 and the fixed
         // 1e-10 floor under -remove_dc, src/io/in.cc:390-398; Nyquist real; atan(0/0) = -pi/2)
         const float *srow = (src_mode == BURG_SRC_VAD && B.use_spec_gain) ? spec + (row0 + f) * B.spitch : nullptr;
@@ -465,9 +467,10 @@ int launch_burg(const BurgParams &B, int src_mode, const BatchDesc &bd, int64_t 
         const int M = B.nfft / 2;
         const size_t bytes_any = (size_t)(ANY64_THREADS / 32) * burg_any_doubles(M) * sizeof(double);
         AnyTables64 tb{B.any_tw, B.any_ts, win, B.nfft, B.log2m};
-        cudaError_t e2 = cudaFuncSetAttribute(k_burg_any, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes_any);
+        auto ka = B.dc1 ? k_burg_any<true> : k_burg_any<false>;
+        cudaError_t e2 = cudaFuncSetAttribute(ka, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes_any);
         lc->begin("k_burg_any", s);
-        if (e2 == cudaSuccess) k_burg_any<<<(unsigned)ntiles, ANY64_THREADS, bytes_any, s>>>(B, src_mode, bd, tb, pcm, spec, ceps, hann);
+        if (e2 == cudaSuccess) ka<<<(unsigned)ntiles, ANY64_THREADS, bytes_any, s>>>(B, src_mode, bd, tb, pcm, spec, ceps, hann);
         lc->end(s);
         if (e2 == cudaSuccess) e2 = cudaGetLastError();
         if (e2 != cudaSuccess) { err = std::string("CUDA: ") + cudaGetErrorString(e2) + " (k_burg_any)"; return CTU_ERR_CUDA; }

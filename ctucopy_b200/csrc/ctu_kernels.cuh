@@ -399,12 +399,24 @@ k_normalise(BatchDesc bd, int dim, int stride, const double *__restrict__ mean, 
     }
 }
 
+// -remove_dc1 in fp64 (src/io/in.cc:343-350): frame t subtracts the mean of the whole ring from the ring, so sample i of
+// frame t - d0 has lost m[t-D] + .. + m[t-d0] by the end of that frame, where frames t-D .. t-d0 are the ones that hold it
+// (i + (d - d0) s < w, and none before frame 0).  `m` points at the mean of frame t (k_dc1_means); the means are subtracted
+// oldest first, in the order the reference's ring takes them.  The sample before frame t, which pre-emphasis reads, is
+// sample s-1 of frame t-1 at d0 = 1 (src/io/in.cc:384).
+__device__ __forceinline__ double dc1_ring_value(double v, const double *__restrict__ m, int i, int d0, int t, int w, int s) {
+    const int D = min(t, d0 + (w - 1 - i) / s);
+    for (int d = D; d >= d0; d--) v -= __ldg(m - d);
+    return v;
+}
+
 // ------------------------------------------------------------------------------------------
 // raw energy (src/io/in.cc:353-361): log of the sum of squares of the frame's raw samples 1..w-1
-// (the first one is skipped).  One warp per frame.
+// (the first one is skipped); under -remove_dc1 the samples as the de-meaned ring holds them (DC1).  One warp per frame.
 // ------------------------------------------------------------------------------------------
+template <bool DC1>
 static __global__ void __launch_bounds__(256)
-k_rawenergy(BatchDesc bd, int window, int wshift, const int16_t *__restrict__ pcm, float *__restrict__ energy) {
+k_rawenergy(BatchDesc bd, int window, int wshift, const int16_t *__restrict__ pcm, float *__restrict__ energy, const double *__restrict__ dc1) {
     const int2 tile = bd.tiles[blockIdx.x];
     const int u = tile.x, t0 = tile.y;
     const int nf = min(DELTA_ROWS_C, bd.nframes[u] - t0);
@@ -412,7 +424,11 @@ k_rawenergy(BatchDesc bd, int window, int wshift, const int16_t *__restrict__ pc
     for (int f = threadIdx.x >> 5; f < nf; f += 8) {
         const int16_t *x = pcm + bd.pcm_off[u] + (int64_t)(t0 + f) * wshift;
         double acc = 0;
-        for (int i = 1 + lane; i < window; i += 32) { const double v = (double)x[i]; acc += v * v; }
+        for (int i = 1 + lane; i < window; i += 32) {
+            double v = (double)x[i];
+            if (DC1) v = dc1_ring_value(v, dc1 + bd.row_off[u] + t0 + f, i, 0, t0 + f, window, wshift);
+            acc += v * v;
+        }
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
         if (lane == 0) energy[bd.row_off[u] + t0 + f] = (float)log(acc);

@@ -50,8 +50,11 @@ struct BurgParams {
     int use_spec_gain;   // VAD source: post-NR spectrum present (gain from d_spec) else own spectrum
     // FFT sizes other than 512: the general kernel k_burg_any (nfft == 0: the specialised k_burg)
     int nfft, log2m;
-    const double2 *any_tw, *any_ts;
     int spitch;          // floats per row of the spectrum matrix
+    const double2 *any_tw, *any_ts;
+    // -remove_dc1: ring means per frame (k_dc1_means), nullptr when off; only k_burg_any applies them (the host routes
+    // -remove_dc1 there at every FFT size)
+    const double *dc1;
 };
 
 struct VadParams {

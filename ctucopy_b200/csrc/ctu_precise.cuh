@@ -263,8 +263,9 @@ k_frames64(const __grid_constant__ FrameParams P, BatchDesc bd, Tables64 tb, con
     }
 }
 
-// The same chain for FFT sizes other than 512: one warp per frame, front end from ctu_any64.cuh.
-template <int SRC, int DST, int KIND>
+// The same chain for FFT sizes other than 512 (and for -remove_dc1 at any size): one warp per frame, front end from
+// ctu_any64.cuh.  DC1: PCM source under -remove_dc1, the frame is built from the de-meaned ring (P.dc1).
+template <int SRC, int DST, int KIND, bool DC1 = false>
 __global__ void __launch_bounds__(ANY64_THREADS)
 k_frames64_any(const __grid_constant__ FrameParams P, BatchDesc bd, Tables64 tb, const int16_t *__restrict__ pcm, const double *__restrict__ src,
                const float *__restrict__ spec, double *__restrict__ dst64, float *__restrict__ dst) {
@@ -287,7 +288,8 @@ k_frames64_any(const __grid_constant__ FrameParams P, BatchDesc bd, Tables64 tb,
             __syncwarp();
         }
         if (SRC == SRC64_PCM) {
-            any64_analysis(z, at, pcm + bd.pcm_off[u] + (int64_t)(t0 + f) * P.wshift, (t0 + f) == 0, P.window, (double)P.preem, P.remove_dc, lane);
+            any64_analysis<DC1>(z, at, pcm + bd.pcm_off[u] + (int64_t)(t0 + f) * P.wshift, (t0 + f) == 0, P.window, (double)P.preem, P.remove_dc, lane,
+                                DC1 ? P.dc1 + row0 + f : nullptr, t0 + f, P.wshift);
             for (int k = lane; k <= M; k += 32) {
                 const cpx<double> X = any64_bin(z, at, k);
                 double pw = X.x * X.x + X.y * X.y;
@@ -312,6 +314,7 @@ static int launch_frames64_t(const FrameParams &P, const BatchDesc &bd, const Ta
     if (tb.nfft) {
         const size_t bytes_any = (size_t)(ANY64_THREADS / 32) * (2 * any64_zslots(tb.nfft / 2) + tb.nfft / 2 + 4 + 128) * sizeof(double);
         auto ka = k_frames64_any<SRC, DST, KIND>;
+        if constexpr (SRC == SRC64_PCM) { if (P.dc1) ka = k_frames64_any<SRC, DST, KIND, true>; }
         cudaError_t e2 = cudaFuncSetAttribute(ka, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes_any);
         if (e2 == cudaSuccess) {
             lc->begin(SRC == SRC64_PCM ? (DST == DST64_FB ? "k_frames64_any<pcm,fb>" : "k_frames64_any<pcm,fea>")

@@ -15,9 +15,11 @@ namespace ctu {
 
 constexpr int SYNANY_THREADS = ANY64_THREADS;  // 4 warps: 4 x (2 zslots(M) + 2M + 4) doubles of shared memory, 135 KB at 2048 points
 
+// DC1: -remove_dc1, the frame is built from the de-meaned ring (dc1 = the ring means of k_dc1_means, one per frame)
+template <bool DC1>
 __global__ void __launch_bounds__(SYNANY_THREADS)
 k_synth_frames_any(int window, int wshift, double preem, int remove_dc, BatchDesc bd, AnyTables64 tb, const int16_t *__restrict__ pcm,
-                   const float *__restrict__ spec, double *__restrict__ yt) {
+                   const float *__restrict__ spec, double *__restrict__ yt, const double *__restrict__ dc1) {
     extern __shared__ __align__(16) double smd[];
     const int lane = threadIdx.x & 31, wv = threadIdx.x >> 5;
     const int nfft = tb.nfft, M = nfft >> 1, nbins = M + 1;
@@ -29,7 +31,7 @@ k_synth_frames_any(int window, int wshift, double preem, int remove_dc, BatchDes
     const int64_t row0 = bd.row_off[u] + t0;
     const int w = window, s = wshift;
     for (int f = wv; f < nf; f += SYNANY_THREADS / 32) {
-        any64_analysis(z, tb, pcm + bd.pcm_off[u] + (int64_t)(t0 + f) * s, (t0 + f) == 0, w, preem, remove_dc, lane);
+        any64_analysis<DC1>(z, tb, pcm + bd.pcm_off[u] + (int64_t)(t0 + f) * s, (t0 + f) == 0, w, preem, remove_dc, lane, DC1 ? dc1 + row0 + f : nullptr, t0 + f, s);
         // ---- real-input split; enhanced magnitude on the original phase, scaled by 1/nfft (src/io/out.cc:417-424) ---
         const float *A = spec + (row0 + f) * tb.spitch;
         const double invn = 1.0 / (double)nfft;
