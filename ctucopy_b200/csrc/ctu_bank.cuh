@@ -132,49 +132,56 @@ __device__ __forceinline__ BankWalk bank_next(const BankWalk &c, const BatchDesc
     return w;
 }
 
-// one tile of the recursion for one bin: 32 frames in shared memory, in place
+// one tile of the recursion: 32 frames in shared memory, in place.  Threads 0-127 own the bin pairs (2t, 2t + 1) and run
+// nr_step2 on packed FP32 with 8-byte loads and stores (SPITCH is even, so every pair is aligned); thread 128 carries bin
+// 256 on the scalar nr_step, in the x half of its state; warps 5-7 have no scan work.
 constexpr int BANK_SCAN_CHUNK = 8;
-// TWO: the warp also carries bin 256 (the 257th bin of 256 threads): all its lanes run that second chain redundantly on
-// the same values -- no divergence, and the two chains of a lane overlap in the pipeline -- and one lane stores it
-template <int MODE, int AKIND, bool FULL, bool TWO>
-__device__ __forceinline__ void bank_scan_chunk(const NrParams &N, ScanState &S, ScanState &S2, float *tile, const uint8_t *fl, int f0, int nf, int t0) {
-    float *x = tile + threadIdx.x;
-    // the bin's values come into registers first (independent loads, all in flight at once); in place, every step would
-    // wait for its own shared-memory load behind the previous step's store
-    float v[BANK_SCAN_CHUNK], b[BANK_SCAN_CHUNK];
+constexpr int BANK_SCAN_PAIRS = 128;
+template <int MODE, int AKIND, bool FULL>
+__device__ __forceinline__ void bank_scan_chunk(const NrParams &N, ScanState2 &S, float *tile, const uint8_t *fl, int f0, int nf, int t0) {
+    cpx<float> *x = reinterpret_cast<cpx<float> *>(tile) + threadIdx.x;
+    // the values come into registers first (independent loads, all in flight at once); in place, every step would wait for
+    // its own shared-memory load behind the previous step's store
+    cpx<float> v[BANK_SCAN_CHUNK];
 #pragma unroll
-    for (int j = 0; j < BANK_SCAN_CHUNK; j++) {
-        v[j] = x[(f0 + j) * SPITCH];
-        if (TWO) b[j] = tile[(f0 + j) * SPITCH + 256];
-    }
+    for (int j = 0; j < BANK_SCAN_CHUNK; j++) v[j] = x[(f0 + j) * (SPITCH / 2)];
 #pragma unroll
     for (int j = 0; j < BANK_SCAN_CHUNK; j++)
-        if (FULL || f0 + j < nf) {
-            const uint8_t g = (MODE != NR_EXTEN) ? fl[f0 + j] : 0;
-            v[j] = nr_step<MODE, AKIND>(N, S, v[j], t0 + f0 + j, g);
-            if (TWO) b[j] = nr_step<MODE, AKIND>(N, S2, b[j], t0 + f0 + j, g);
-        }
+        if (FULL || f0 + j < nf) v[j] = nr_step2<MODE, AKIND>(N, S, v[j], t0 + f0 + j, (MODE != NR_EXTEN) ? fl[f0 + j] : 0);
 #pragma unroll
-    for (int j = 0; j < BANK_SCAN_CHUNK; j++) {
-        x[(f0 + j) * SPITCH] = v[j];
-        if (TWO && (threadIdx.x & 31) == 31) tile[(f0 + j) * SPITCH + 256] = b[j];
-    }
+    for (int j = 0; j < BANK_SCAN_CHUNK; j++) x[(f0 + j) * (SPITCH / 2)] = v[j];
+}
+template <int MODE, int AKIND, bool FULL>
+__device__ __forceinline__ void bank_scan_chunk_last(const NrParams &N, ScanState2 &S2, float *tile, const uint8_t *fl, int f0, int nf, int t0) {
+    float *x = tile + 2 * BANK_SCAN_PAIRS;
+    ScanState S;
+    S.Navg = S2.Navg.x; S.Yavg = S2.Yavg.x; S.Nravg = S2.Nravg.x;
+    float v[BANK_SCAN_CHUNK];
+#pragma unroll
+    for (int j = 0; j < BANK_SCAN_CHUNK; j++) v[j] = x[(f0 + j) * SPITCH];
+#pragma unroll
+    for (int j = 0; j < BANK_SCAN_CHUNK; j++)
+        if (FULL || f0 + j < nf) v[j] = nr_step<MODE, AKIND>(N, S, v[j], t0 + f0 + j, (MODE != NR_EXTEN) ? fl[f0 + j] : 0);
+#pragma unroll
+    for (int j = 0; j < BANK_SCAN_CHUNK; j++) x[(f0 + j) * SPITCH] = v[j];
+    S2.Navg.x = S.Navg; S2.Yavg.x = S.Yavg; S2.Nravg.x = S.Nravg;
 }
 
 template <int MODE, int AKIND>
-__device__ __forceinline__ void bank_scan_tile(const NrParams &N, ScanState &S, ScanState &S2, float *tile, const uint8_t *fl, int nf, int t0) {
-    const bool last_warp = (threadIdx.x >> 5) == BANK_THREADS / 32 - 1;            // warp-uniform
+__device__ __forceinline__ void bank_scan_tile(const NrParams &N, ScanState2 &S, float *tile, const uint8_t *fl, int nf, int t0) {
     // eight frames at a time; the loop over the chunks stays rolled (unrolled over all 32 frames, seven mode variants made
     // the kernel 240 KB of code).  Whole chunks take the branch-free body.
+    if (threadIdx.x < BANK_SCAN_PAIRS) {
 #pragma unroll 1
-    for (int f0 = 0; f0 < nf; f0 += BANK_SCAN_CHUNK) {
-        const bool full = f0 + BANK_SCAN_CHUNK <= nf;
-        if (last_warp) {
-            if (full) bank_scan_chunk<MODE, AKIND, true, true>(N, S, S2, tile, fl, f0, nf, t0);
-            else bank_scan_chunk<MODE, AKIND, false, true>(N, S, S2, tile, fl, f0, nf, t0);
-        } else {
-            if (full) bank_scan_chunk<MODE, AKIND, true, false>(N, S, S2, tile, fl, f0, nf, t0);
-            else bank_scan_chunk<MODE, AKIND, false, false>(N, S, S2, tile, fl, f0, nf, t0);
+        for (int f0 = 0; f0 < nf; f0 += BANK_SCAN_CHUNK) {
+            if (f0 + BANK_SCAN_CHUNK <= nf) bank_scan_chunk<MODE, AKIND, true>(N, S, tile, fl, f0, nf, t0);
+            else bank_scan_chunk<MODE, AKIND, false>(N, S, tile, fl, f0, nf, t0);
+        }
+    } else if (threadIdx.x == BANK_SCAN_PAIRS) {
+#pragma unroll 1
+        for (int f0 = 0; f0 < nf; f0 += BANK_SCAN_CHUNK) {
+            if (f0 + BANK_SCAN_CHUNK <= nf) bank_scan_chunk_last<MODE, AKIND, true>(N, S, tile, fl, f0, nf, t0);
+            else bank_scan_chunk_last<MODE, AKIND, false>(N, S, tile, fl, f0, nf, t0);
         }
     }
 }
@@ -212,8 +219,8 @@ k_bank(const __grid_constant__ BankParams B, BatchDesc bd, int ntiles, int u0, i
         mbar_expect_tx(bar, bytes);
         bulk_g2s(tile, spec + (cur.row0 + cur.t0) * SPITCH, bytes, bar);
     }
-    ScanState S, S2;
-    S.Navg = S2.Navg = 0.f; S.Yavg = S2.Yavg = 0.f; S.Nravg = S2.Nravg = 0.f; S.Nd = S2.Nd = 0.0; S.Yd = S2.Yd = 0.0;
+    ScanState2 S;
+    S.Navg = S.Yavg = S.Nravg = mk(0.f, 0.f);
 #pragma unroll 1
     for (int it = 0; cur.valid; it++) {
         const BankWalk nxt = bank_next<NR>(cur, bd, ntiles, u0, n_utts);
@@ -226,15 +233,15 @@ k_bank(const __grid_constant__ BankParams B, BatchDesc bd, int ntiles, int u0, i
                 // exten: smoothed noise / speech start at 0.95 / 0.05 (src/nr/nr.cc:86-93); *ss: the noise estimate of a
                 // standalone file starts at 0 (src/nr/nr.cc:212-222)
                 const float n0 = (B.nr.mode == NR_EXTEN) ? 0.95f : 0.f;
-                S.Navg = S2.Navg = n0; S.Yavg = S2.Yavg = 0.05f; S.Nravg = S2.Nravg = 0.f;
+                S.Navg = mk(n0, n0); S.Yavg = mk(0.05f, 0.05f); S.Nravg = mk(0.f, 0.f);
             }
             if (B.nr.mode != NR_EXTEN) __syncthreads();                      // flags staged
             const bool a2 = B.nr.a_kind == 2;
             switch (B.nr.mode) {
-                case NR_EXTEN: if (a2) bank_scan_tile<NR_EXTEN, 2>(B.nr, S, S2, tile, sFlags, nf, cur.t0); else bank_scan_tile<NR_EXTEN, 1>(B.nr, S, S2, tile, sFlags, nf, cur.t0); break;
-                case NR_HWSS: if (a2) bank_scan_tile<NR_HWSS, 2>(B.nr, S, S2, tile, sFlags, nf, cur.t0); else bank_scan_tile<NR_HWSS, 1>(B.nr, S, S2, tile, sFlags, nf, cur.t0); break;
-                case NR_FWSS: if (a2) bank_scan_tile<NR_FWSS, 2>(B.nr, S, S2, tile, sFlags, nf, cur.t0); else bank_scan_tile<NR_FWSS, 1>(B.nr, S, S2, tile, sFlags, nf, cur.t0); break;
-                default: bank_scan_tile<NR_2FWSS, 1>(B.nr, S, S2, tile, sFlags, nf, cur.t0); break;
+                case NR_EXTEN: if (a2) bank_scan_tile<NR_EXTEN, 2>(B.nr, S, tile, sFlags, nf, cur.t0); else bank_scan_tile<NR_EXTEN, 1>(B.nr, S, tile, sFlags, nf, cur.t0); break;
+                case NR_HWSS: if (a2) bank_scan_tile<NR_HWSS, 2>(B.nr, S, tile, sFlags, nf, cur.t0); else bank_scan_tile<NR_HWSS, 1>(B.nr, S, tile, sFlags, nf, cur.t0); break;
+                case NR_FWSS: if (a2) bank_scan_tile<NR_FWSS, 2>(B.nr, S, tile, sFlags, nf, cur.t0); else bank_scan_tile<NR_FWSS, 1>(B.nr, S, tile, sFlags, nf, cur.t0); break;
+                default: bank_scan_tile<NR_2FWSS, 1>(B.nr, S, tile, sFlags, nf, cur.t0); break;
             }
             __syncthreads();
         }
@@ -295,15 +302,33 @@ k_bank(const __grid_constant__ BankParams B, BatchDesc bd, int ntiles, int u0, i
         } else {
             const float *y = sY + lane * B.ypitch;
             if (KIND == KIND_DCTC) {
-                for (int i = wv; i < B.nrows; i += BANK_THREADS / 32) {
+                // rows i and i + 8 in one pass over the band vector: each 16-byte read of y (four wavefronts: every lane its
+                // own frame) feeds two rows, whose matrix reads are broadcasts; pad taps are zero, pad y entries are zero
+                const float4 *y4 = reinterpret_cast<const float4 *>(y);
+                constexpr int NW = BANK_THREADS / 32;
+                for (int i = wv; i < B.nrows; i += 2 * NW) {
                     const float4 *m4 = reinterpret_cast<const float4 *>(sM + i * B.nbp);
-                    const float4 *y4 = reinterpret_cast<const float4 *>(y);
                     cpx<float> a01 = mk<float>(0.f, 0.f), a23 = a01;
+                    if (i + NW < B.nrows) {                                    // warp-uniform
+                        const float4 *n4 = reinterpret_cast<const float4 *>(sM + (i + NW) * B.nbp);
+                        cpx<float> b01 = a01, b23 = a01;
+                        // unrolled four times, k_bank<dctc, fea, nr> spills
+#pragma unroll 2
+                        for (int q = 0; q < B.nbp / 4; q++) {
+                            const float4 v = y4[q], m = m4[q], n = n4[q];
+                            a01 = pfma(mk<float>(v.x, v.y), mk<float>(m.x, m.y), a01);
+                            a23 = pfma(mk<float>(v.z, v.w), mk<float>(m.z, m.w), a23);
+                            b01 = pfma(mk<float>(v.x, v.y), mk<float>(n.x, n.y), b01);
+                            b23 = pfma(mk<float>(v.z, v.w), mk<float>(n.z, n.w), b23);
+                        }
+                        sO[lane * od + i + NW] = (b01.x + b01.y) + (b23.x + b23.y);
+                    } else {
 #pragma unroll 4
-                    for (int q = 0; q < B.nbp / 4; q++) {                      // pad taps are zero, pad y entries are zero
-                        const float4 v = y4[q], m = m4[q];
-                        a01 = pfma(mk<float>(v.x, v.y), mk<float>(m.x, m.y), a01);
-                        a23 = pfma(mk<float>(v.z, v.w), mk<float>(m.z, m.w), a23);
+                        for (int q = 0; q < B.nbp / 4; q++) {
+                            const float4 v = y4[q], m = m4[q];
+                            a01 = pfma(mk<float>(v.x, v.y), mk<float>(m.x, m.y), a01);
+                            a23 = pfma(mk<float>(v.z, v.w), mk<float>(m.z, m.w), a23);
+                        }
                     }
                     sO[lane * od + i] = (a01.x + a01.y) + (a23.x + a23.y);
                 }

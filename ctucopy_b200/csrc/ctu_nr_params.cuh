@@ -195,6 +195,65 @@ __device__ __forceinline__ float nr_step(const NrParams &N, ScanState &S, float 
     return xi;
 }
 
+// recursion state of two bins (x: bin 2t, y: bin 2t + 1)
+struct ScanState2 { cpx<float> Navg, Yavg, Nravg; };
+
+// nr_step on two bins at once, for the fused scan of k_bank.  Each lane runs the operations that nr_step compiles to, in
+// the same order and with the same contractions (nvcc turns xi - b * Navg into fma(-Navg, b, xi)), on packed FP32
+// (FADD2 / FMUL2 / FFMA2, ctu_fft.cuh), which rounds every lane like the scalar instruction: the results are nr_step's bit
+// for bit.  Reciprocals, square roots and compares stay scalar, one per lane.  The general exponent (AKIND 0) never
+// reaches the fused scan.
+template <int MODE, int AKIND>
+__device__ __forceinline__ cpx<float> nr_step2(const NrParams &N, ScanState2 &S, cpx<float> xi, int t, uint8_t flag) {
+    static_assert(AKIND == 1 || AKIND == 2, "nr_step2: a == 1 or a == 2");
+    const float p = N.p, q = 1.f - N.p;
+    const cpx<float> pp = mk(p, p), qq = mk(q, q);
+    if (MODE == NR_EXTEN) {
+        cpx<float> H, omH;
+        if (AKIND == 1) {
+            const cpx<float> s = S.Navg + S.Yavg;
+            const cpx<float> r = mk(fast_rcp(s.x), fast_rcp(s.y));
+            H = pmul(S.Navg, r); omH = pmul(S.Yavg, r);
+        } else {
+            const cpx<float> y2 = pmul(S.Yavg, S.Yavg);
+            const cpx<float> h2 = pfma(S.Navg, S.Navg, y2);
+            const cpx<float> ri = mk(fast_rsqrt(h2.x), fast_rsqrt(h2.y));
+            const cpx<float> hh = pmul(h2, ri);
+            H = pmul(S.Navg, ri);
+            const cpx<float> den = pmul(hh, hh + S.Navg);
+            omH = pmul(y2, mk(fast_rcp(den.x), fast_rcp(den.y)));
+        }
+        const cpx<float> Nn = pmul(H, xi);
+        S.Navg = pfma(pp, S.Navg, pmul(qq, Nn));
+        const cpx<float> d = xi - S.Navg;
+        // a == 2 uses Yavg only squared, and d * d == |d| * |d| exactly: the sign stays
+        S.Yavg = (AKIND == 1) ? mk(fabsf(d.x), fabsf(d.y)) : d;
+        return pmul(xi, omH);
+    }
+    const int ninit = (MODE == NR_HWSS) ? N.initsegs - (t + 1) : N.initsegs - t;
+    const bool upd = (flag == 0) || ninit > 0;
+    if (MODE == NR_2FWSS) {
+        if (upd) S.Navg = pfma(pp, S.Navg, pmul(qq, xi));
+        xi = xi - S.Navg;
+        xi = mk(fabsf(xi.x), fabsf(xi.y));
+        if (upd) S.Nravg = pfma(pp, S.Nravg, pmul(qq, xi));
+        xi = xi - S.Nravg;
+        return mk(fabsf(xi.x), fabsf(xi.y));
+    }
+    if (AKIND == 2) xi = pmul(xi, xi);
+    if (upd) S.Navg = pfma(pp, S.Navg, pmul(qq, xi));
+    xi = pfma(S.Navg, mk(-N.b, -N.b), xi);
+    if (MODE == NR_HWSS) {
+        if (xi.x < 0.f) xi.x = 0.f;
+        if (xi.y < 0.f) xi.y = 0.f;
+    } else {
+        if (xi.x < 0.f) xi.x = -xi.x;
+        if (xi.y < 0.f) xi.y = -xi.y;
+    }
+    if (AKIND == 2) xi = mk(sqrtf(xi.x), sqrtf(xi.y));
+    return xi;
+}
+
 // ------------------------------------------------------------------------------------------
 // shared front end in double precision for one frame held by a 16-thread group
 // ------------------------------------------------------------------------------------------

@@ -57,7 +57,7 @@ def main():
         elif cur and re.match(r"\s+/\*[0-9a-f]{4,5}\*/", ln):
             funcs[cur].append(re.sub(r"/\* 0x[0-9a-f]+ \*/", "", ln).rstrip())
     want = [("k_frames2ILi400ELb0", ["FADD2", "FMUL2", "FFMA2", "LDGSTS", "SHFL", "STG", "LDS.64", "BAR"]),
-            ("k_bankILi3ELi2ELb1", ["UBLKCP", "SYNCS", "FFMA2", "LDS.128", "MUFU", "BAR", "STG"]),
+            ("k_bankILi3ELi2ELb1", ["UBLKCP", "SYNCS", "FADD2", "FMUL2", "FFMA2", "LDS.64", "STS.64", "LDS.128", "MUFU", "BAR", "STG"]),
             ("k_bankILi3ELi2ELb0", ["UBLKCP", "SYNCS", "FFMA2", "LDS.128", "BAR", "STG"]),
             ("k_trapdctILi51ELi8", ["FFMA2", "FADD2", "LDCU.128", "LDS"]),
             ("k_frames256", ["FADD2", "FFMA2", "LDGSTS", "SHFL"]),
